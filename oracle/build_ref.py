@@ -1,6 +1,7 @@
 """Build oracle/_ref: the reference's OWN CPU rotated-IoU (utils/detzero_utils/ops/iou3d_nms/src/iou3d_cpu.cpp) compiled from the
-sources where they lie under /root/reference (never copied), plus a 10-line pybind11 binding of ours.  Used to pin the
-oracle's rotated-IoU restatement (tests/test_oracle.py).  g++ directly; outputs only into oracle/_ref/ (git-ignored)."""
+sources where they lie in the reference checkout (REF_SRC; never copied), plus a 10-line pybind11 binding of ours.  Used by
+tests/golden/make_golden_host.py to record the output that pins the oracle's rotated-IoU restatement.  g++ directly; outputs
+only into oracle/_ref/ (git-ignored)."""
 import os
 import subprocess
 import sys

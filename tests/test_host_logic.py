@@ -154,29 +154,13 @@ def test_frame_file_format_and_result_pkl(tmp_path):
 
 
 def test_merge_sweeps_restatement_matches_reference_source():
-    """the oracle's merge_sweeps against the reference's own DatasetTemplate.merge_sweeps, imported from /root/reference when mounted"""
-    import numpy as np
+    """the oracle's merge_sweeps against the output of the reference's own DatasetTemplate.merge_sweeps statements
+    (detection/detzero_det/datasets/dataset.py) on the same inputs, stored by tests/golden/make_golden_host.py"""
     import os
+    import numpy as np
     from oracle import det_ref
-    if not os.path.isdir('/root/reference'):
-        pytest.skip('/root/reference not mounted')
-    import importlib.util
-    import re
-    src = open('/root/reference/detection/detzero_det/datasets/dataset.py').read()
-    m = re.search(r'    @staticmethod\n    def merge_sweeps\(.*?\n        return point_clouds\n', src, re.S)
-    ns = {'np': np}
-    exec('class _T:\n' + m.group(0), ns)                            # the reference's own statements, executed as they are
-    g = np.random.default_rng(3)
-
-    def pose():
-        a = g.uniform(-0.2, 0.2)
-        p = np.eye(4); p[:2, :2] = [[np.cos(a), -np.sin(a)], [np.sin(a), np.cos(a)]]; p[:3, 3] = g.uniform(-3, 3, 3)
-        return p
-    infos = [{'pose': pose(), 'time_stamp': 1550000000000000 - 100000 * k} for k in range(3)]
-    pts = []
-    for k in range(3):
-        a = g.normal(0, 20, (500, 6)).astype(np.float32); a[:, 5] = np.where(g.random(500) < 0.9, -1, 1)
-        pts.append(a)
-    want = ns['_T'].merge_sweeps(infos[0], infos, [p.copy() for p in pts])
-    got = det_ref.merge_sweeps(infos[0], infos, [p.copy() for p in pts])
+    from tests import util
+    want = np.load(os.path.join(os.path.dirname(os.path.abspath(__file__)), 'golden', 'host.npz'))['merge_sweeps']
+    infos, pts = util.merge_sweeps_inputs()
+    got = det_ref.merge_sweeps(infos[0], infos, pts)
     assert np.array_equal(want, got)

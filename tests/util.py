@@ -40,6 +40,30 @@ def clustered_cloud(n, seed, pc_range=SMALL_RANGE, c=5):
     return np.concatenate([p, f], axis=1).astype(np.float32)
 
 
+def merge_sweeps_inputs(seed=3):
+    """three sweeps of 500 points (x y z intensity elongation NLZ-flag, 90 % NLZ == -1), small-angle poses, 0.1 s apart"""
+    g = np.random.default_rng(seed)
+
+    def pose():
+        a = g.uniform(-0.2, 0.2)
+        p = np.eye(4); p[:2, :2] = [[np.cos(a), -np.sin(a)], [np.sin(a), np.cos(a)]]; p[:3, 3] = g.uniform(-3, 3, 3)
+        return p
+    infos = [{'pose': pose(), 'time_stamp': 1550000000000000 - 100000 * k} for k in range(3)]
+    pts = []
+    for k in range(3):
+        a = g.normal(0, 20, (500, 6)).astype(np.float32); a[:, 5] = np.where(g.random(500) < 0.9, -1, 1)
+        pts.append(a)
+    return infos, pts
+
+
+def iou_boxes(seed=7, n=300):
+    """rotated boxes (x y z dx dy dz heading); boxes 100..199 sit within ~0.2 m of boxes 0..99, so many pairs overlap partly"""
+    g = np.random.default_rng(seed)
+    b = np.concatenate([g.uniform(-10, 10, (n, 3)), g.uniform(1, 5, (n, 3)), g.uniform(-3.2, 3.2, (n, 1))], 1).astype(np.float32)
+    b[100:200, :2] = b[:100, :2] + g.normal(0, 0.2, (100, 2)).astype(np.float32)
+    return b
+
+
 from detzero_b200.synthetic import model_cfg, CLASS_NAMES    # noqa: E402,F401  (one definition, shared with bench.py)
 
 
