@@ -41,6 +41,9 @@ _SIGS = {
     'dz_rulebook_conv': (ci, [vp, vp, ci, ci, vp, vp, vp, vp, vp, vp, vp, vp, vp, ci, vp, vp, vp, vp, vp, sz, vp, ci, vp]),
     'dz_rulebook_schedule_ws_bytes': (sz, [ci]),
     'dz_rulebook_schedule': (ci, [vp, ci, vp, vp, vp, sz, ci, ci, ci, vp, vp]),
+    'dz_rulebook_subm_masks': (ci, [vp, vp, ci, ci, ci, ci, ci, vp, vp, vp, vp, vp, ci, ci, vp]),
+    'dz_rulebook_conv_masks': (ci, [vp, vp, ci, ci, vp, vp, vp, vp, vp, vp, vp, vp, vp, ci, vp, vp, vp, sz, vp, ci, vp]),
+    'dz_rulebook_schedule_direct': (ci, [vp, ci, vp, ci, vp, vp, vp, vp, ci, vp, vp, vp, vp, vp, sz, ci, vp, vp]),
     'dz_spconv_fwd': (ci, [vp, ci, ci, vp, ci, ci, vp, vp, ci, vp, vp, vp, vp, ci, vp, ci, ci, vp]),
     'dz_rulebook_transpose': (ci, [vp, ci, ci, vp, vp, ci, vp]),
     'dz_spconv_wgrad': (ci, [vp, ci, vp, ci, ci, vp, ci, vp, ci, vp, vp]),

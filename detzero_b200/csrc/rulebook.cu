@@ -47,8 +47,18 @@ __device__ __forceinline__ uint32_t sched_digest(uint32_t m, int K) {
     return (~d) & (SCHED_BINS - 1);
 }
 
-// one table row: v[0..K-1] neighbour rows (or -1).  s_hist: the block's digest histogram in shared memory (hot digests
-// are shared by thousands of rows: per-row or per-warp global atomics on them serialise in L2)
+// one row's schedule digest + mask.  s_hist: the block's digest histogram in shared memory (hot digests are shared by
+// thousands of rows: per-row or per-warp global atomics on them serialise in L2)
+__device__ __forceinline__ void sched_emit(const TableOut& to, bool valid, int i, uint32_t mask, int K, int* s_hist, int frame) {
+    if (to.keys && valid) {
+        const uint32_t key = sched_key(to, sched_digest(mask, K), frame);
+        to.keys[i] = (uint16_t)key;
+        to.masks[i] = (int)mask;
+        atomicAdd(s_hist + key, 1);
+    }
+}
+
+// one table row: v[0..K-1] neighbour rows (or -1)
 __device__ __forceinline__ void table_emit(const TableOut& to, bool valid, int i, int cap, const int (&v)[27], int K, int* s_hist, int frame) {
     uint32_t mask = 0;
 #pragma unroll
@@ -69,12 +79,7 @@ __device__ __forceinline__ void table_emit(const TableOut& to, bool valid, int i
             dst[7] = make_int4(0, 0, 0, 0);
         }
     }
-    if (to.keys && valid) {
-        const uint32_t key = sched_key(to, sched_digest(mask, K), frame);
-        to.keys[i] = (uint16_t)key;
-        to.masks[i] = (int)mask;
-        atomicAdd(s_hist + key, 1);
-    }
+    sched_emit(to, valid, i, mask, K, s_hist, frame);
 }
 
 // the last block to finish turns the digest histogram into exclusive offsets (block of 256 threads, 32 bins each)
@@ -264,17 +269,115 @@ __global__ void __launch_bounds__(256) k_conv_nbr(const int32_t* __restrict__ ou
     table_finish(to, s_hist);
 }
 
+// ---- direct path: neighbour masks line by line, no table ------------------------------------------------------------
+// With a dilation of 1 the KW x-taps of one (kz, ky) kernel line are KW <= 3 adjacent cells of one lattice row, so one or two
+// bitmap words hold all of them: one dependent load per line instead of one bitmap -> prefix -> perm chain per tap.  The
+// x range is clipped to [0, W) first, so bits of the neighbouring x-row, of the frame's cells_pad tail or of the next word
+// never enter (the same per-dimension bounds as grid_lookup).  Tap (kz, ky, kx) of output site (z, y, x) reads input cell
+// (z*s - p + kz, y*s - p + ky, x*s - p + kx); a submanifold conv is s = 1, p = (k-1)/2.
+struct LineWords {
+    long long c_lo;                                 // first in-range cell of the line
+    uint32_t w_lo, w_hi;                            // bitmap words of the first / last in-range cell (equal if one word)
+    int x_lo, n;                                    // first in-range tap index kx, number of in-range taps (0: line outside)
+};
+__device__ __forceinline__ LineWords line_words(const GridIndex& g, int b, int z, int y, int x0, int KW) {
+    LineWords l{0, 0, 0, 0, 0};
+    if ((unsigned)z >= (unsigned)g.D || (unsigned)y >= (unsigned)g.H) return l;
+    const int xlo = max(x0, 0), xhi = min(x0 + KW - 1, g.W - 1);
+    if (xlo > xhi) return l;
+    l.c_lo = (long long)b * g.cells_pad + ((long long)z * g.H + y) * g.W + xlo;
+    const long long c_hi = l.c_lo + (xhi - xlo);
+    l.w_lo = __ldg(g.bitmap + (l.c_lo >> 5));
+    l.w_hi = (c_hi >> 5) != (l.c_lo >> 5) ? __ldg(g.bitmap + (c_hi >> 5)) : l.w_lo;
+    l.x_lo = xlo - x0;
+    l.n = xhi - xlo + 1;
+    return l;
+}
+// bits 0..n-1 = cells c_lo .. c_lo+n-1 are active (the 64-bit window w_hi:w_lo starts at c_lo's word)
+__device__ __forceinline__ uint32_t line_bits(const LineWords& l) {
+    const unsigned long long win = ((unsigned long long)l.w_hi << 32) | l.w_lo;
+    return (uint32_t)(win >> (l.c_lo & 31)) & ((1u << l.n) - 1u);
+}
+
+// 27-bit neighbour mask of one output site (the centre tap of a submanifold conv is the site itself: always live)
+__device__ __forceinline__ uint32_t site_mask(const GridIndex& g, const ConvGeom& cg, int4 c, int centre) {
+    const int z0 = c.y * cg.s[0] - cg.p[0], y0 = c.z * cg.s[1] - cg.p[1], x0 = c.w * cg.s[2] - cg.p[2];
+    uint32_t m = 0;
+#pragma unroll
+    for (int kz = 0; kz < 3; ++kz)
+#pragma unroll
+        for (int ky = 0; ky < 3; ++ky)
+            if (kz < cg.k[0] && ky < cg.k[1]) {
+                const LineWords l = line_words(g, c.x, z0 + kz, y0 + ky, x0, cg.k[2]);
+                if (l.n) m |= line_bits(l) << ((kz * cg.k[1] + ky) * cg.k[2] + l.x_lo);
+            }
+    if (centre >= 0) m |= 1u << centre;
+    return m;
+}
+
+// mask pass: masks[i], keys[i] and the digest histogram exactly as table_emit leaves them, no table.  perm_walk (a
+// submanifold conv on an index with perm): thread r takes row perm[r], i.e. rows in lattice order, so the lanes of a warp
+// probe neighbouring cells and share bitmap lines (the rows themselves are in the voxelizer's first-appearance order).
+__device__ __forceinline__ void mask_rows(const int32_t* __restrict__ coords, int n, const ConvGeom& cg, const GridIndex& g, int centre,
+                                          const int32_t* __restrict__ perm_walk, const TableOut& to, int* s_hist) {
+    const int K = cg.k[0] * cg.k[1] * cg.k[2];
+    for (int r = blockIdx.x * blockDim.x + threadIdx.x; r < n; r += gridDim.x * blockDim.x) {
+        const int i = perm_walk ? __ldg(perm_walk + r) : r;
+        const int4 c = __ldg(reinterpret_cast<const int4*>(coords) + i);    // b,z,y,x
+        sched_emit(to, true, i, site_mask(g, cg, c, centre), K, s_hist, c.x);
+    }
+}
+__global__ void __launch_bounds__(256) k_subm_mask(const int32_t* __restrict__ coords, const int* __restrict__ d_n, int cap, ConvGeom cg,
+                                                   GridIndex g, int centre, const int32_t* __restrict__ perm_walk, TableOut to) {
+    __shared__ int s_hist[SCHED_BINS];
+    for (int b = threadIdx.x; b < SCHED_BINS; b += blockDim.x) s_hist[b] = 0;
+    __syncthreads();
+    mask_rows(coords, min(*d_n, cap), cg, g, centre, perm_walk, to, s_hist);
+    table_finish(to, s_hist);
+}
+__global__ void __launch_bounds__(256) k_conv_mask(const int32_t* __restrict__ out_coords, const int* __restrict__ d_n_out, int out_cap,
+                                                   ConvGeom cg, GridIndex gin, TableOut to) {
+    __shared__ int s_hist[SCHED_BINS];
+    for (int b = threadIdx.x; b < SCHED_BINS; b += blockDim.x) s_hist[b] = 0;
+    __syncthreads();
+    mask_rows(out_coords, min(*d_n_out, out_cap), cg, gin, -1, nullptr, to, s_hist);
+    table_finish(to, s_hist);
+}
+
+static ConvGeom subm_geom(int D, int H, int W, const int* ks) {
+    ConvGeom cg;
+    const int dhw[3] = {D, H, W};
+    for (int d = 0; d < 3; ++d) { cg.k[d] = ks[d]; cg.s[d] = 1; cg.p[d] = (ks[d] - 1) / 2; cg.in_dhw[d] = cg.out_dhw[d] = dhw[d]; }
+    return cg;
+}
+
+extern "C" int dz_rulebook_subm_masks(const int32_t* coords, const int* d_n, int cap, int B, int D, int H, int W, const int* ks,
+                                      const uint32_t* bitmap, const uint32_t* prefix, const int32_t* perm, void* sched_ws,
+                                      int sched_frame_major, int perm_walk, dz_stream_t stream) {
+    DZ_CHECK_ARG(coords && d_n && bitmap && prefix && sched_ws && cap >= 1 && (perm || !perm_walk));
+    DZ_CHECK_ARG(ks[0] % 2 == 1 && ks[1] % 2 == 1 && ks[2] % 2 == 1 && ks[0] <= 3 && ks[1] <= 3 && ks[2] <= 3);
+    TableOut to = table_out(nullptr, nullptr, sched_ws, cap, B, sched_frame_major);
+    DZ_CUDA(cudaMemsetAsync(sched_ws, 0, sched_zero_bytes(cap), (cudaStream_t)stream));
+    GridIndex g{bitmap, prefix, perm, B, D, H, W, dz_cells_pad(D, H, W)};
+    const int blocks = max(1, min(dz_cdiv(cap, 256), DZ_NUM_SMS * 8));
+    k_subm_mask<<<blocks, 256, 0, (cudaStream_t)stream>>>(coords, d_n, cap, subm_geom(D, H, W, ks), g, (ks[0] * ks[1] * ks[2] - 1) / 2,
+                                                           perm_walk ? perm : nullptr, to);
+    DZ_LAUNCH_CHECK();
+    return DZ_OK;
+}
+
 __global__ void k_clamp_count(int* d_n, int cap) {
     if (threadIdx.x == 0 && blockIdx.x == 0 && *d_n > cap) *d_n = cap;   // overflow is reported by the host wrapper
 }
 
-extern "C" int dz_rulebook_conv(const int32_t* in_coords, const int* d_n_in, int in_cap, int B, const int* in_dhw,
-                                const int* ks, const int* st_, const int* pd, const uint32_t* in_bitmap,
-                                const uint32_t* in_prefix, const int32_t* in_perm, int32_t* out_coords, int* d_n_out,
-                                int out_cap, uint32_t* out_bitmap, uint32_t* out_prefix, int32_t* nbr, int32_t* tab, void* ws,
-                                size_t ws_bytes, void* sched_ws, int sched_frame_major, dz_stream_t stream) {
-    DZ_CHECK_ARG(in_coords && d_n_in && in_bitmap && in_prefix && out_coords && d_n_out && out_bitmap && out_prefix && (nbr || tab));
-    DZ_CHECK_ARG(!sched_ws || tab);
+// the strided conv with a table (nbr / tab) or, masks_only, the direct path's mask pass (sched_ws, no table)
+static int rulebook_conv(const int32_t* in_coords, const int* d_n_in, int in_cap, int B, const int* in_dhw,
+                         const int* ks, const int* st_, const int* pd, const uint32_t* in_bitmap,
+                         const uint32_t* in_prefix, const int32_t* in_perm, int32_t* out_coords, int* d_n_out,
+                         int out_cap, uint32_t* out_bitmap, uint32_t* out_prefix, int32_t* nbr, int32_t* tab, void* ws,
+                         size_t ws_bytes, void* sched_ws, int sched_frame_major, bool masks_only, dz_stream_t stream) {
+    DZ_CHECK_ARG(in_coords && d_n_in && in_bitmap && in_prefix && out_coords && d_n_out && out_bitmap && out_prefix);
+    DZ_CHECK_ARG(masks_only ? (sched_ws && !nbr && !tab) : ((nbr || tab) && (!sched_ws || tab)));
     DZ_CHECK_ARG(in_cap >= 1 && out_cap >= 1 && B >= 1);
     ConvGeom cg;
     for (int d = 0; d < 3; ++d) {
@@ -297,9 +400,28 @@ extern "C" int dz_rulebook_conv(const int32_t* in_coords, const int* d_n_in, int
     int blocks_out = max(1, min(dz_cdiv(out_cap, 256), DZ_NUM_SMS * 8));
     TableOut to = table_out(nbr, tab, sched_ws, out_cap, B, sched_frame_major);
     if (sched_ws) DZ_CUDA(cudaMemsetAsync(sched_ws, 0, sched_zero_bytes(out_cap), st));
-    k_conv_nbr<<<blocks_out, 256, 0, st>>>(out_coords, d_n_out, out_cap, cg, gin, to);
+    if (masks_only) k_conv_mask<<<blocks_out, 256, 0, st>>>(out_coords, d_n_out, out_cap, cg, gin, to);
+    else k_conv_nbr<<<blocks_out, 256, 0, st>>>(out_coords, d_n_out, out_cap, cg, gin, to);
     DZ_LAUNCH_CHECK();
     return DZ_OK;
+}
+
+extern "C" int dz_rulebook_conv(const int32_t* in_coords, const int* d_n_in, int in_cap, int B, const int* in_dhw,
+                                const int* ks, const int* st_, const int* pd, const uint32_t* in_bitmap,
+                                const uint32_t* in_prefix, const int32_t* in_perm, int32_t* out_coords, int* d_n_out,
+                                int out_cap, uint32_t* out_bitmap, uint32_t* out_prefix, int32_t* nbr, int32_t* tab, void* ws,
+                                size_t ws_bytes, void* sched_ws, int sched_frame_major, dz_stream_t stream) {
+    return rulebook_conv(in_coords, d_n_in, in_cap, B, in_dhw, ks, st_, pd, in_bitmap, in_prefix, in_perm, out_coords, d_n_out, out_cap,
+                         out_bitmap, out_prefix, nbr, tab, ws, ws_bytes, sched_ws, sched_frame_major, false, stream);
+}
+
+extern "C" int dz_rulebook_conv_masks(const int32_t* in_coords, const int* d_n_in, int in_cap, int B, const int* in_dhw,
+                                      const int* ks, const int* st_, const int* pd, const uint32_t* in_bitmap,
+                                      const uint32_t* in_prefix, const int32_t* in_perm, int32_t* out_coords, int* d_n_out,
+                                      int out_cap, uint32_t* out_bitmap, uint32_t* out_prefix, void* ws, size_t ws_bytes,
+                                      void* sched_ws, int sched_frame_major, dz_stream_t stream) {
+    return rulebook_conv(in_coords, d_n_in, in_cap, B, in_dhw, ks, st_, pd, in_bitmap, in_prefix, in_perm, out_coords, d_n_out, out_cap,
+                         out_bitmap, out_prefix, nullptr, nullptr, ws, ws_bytes, sched_ws, sched_frame_major, true, stream);
 }
 
 
@@ -320,7 +442,9 @@ extern "C" int dz_rulebook_conv(const int32_t* in_coords, const int* d_n_in, int
 // The table itself stays in canonical row order (row-major, one 128-byte line per row); the conv kernel reads row
 // order[p].  Every row's accumulation order over k is unchanged, so results are bit-identical to the unscheduled launch.
 // =====================================================================================================================
-static constexpr int SCHED_CHUNK = 512;            // rows per scatter block
+// rows per scatter block: each block zeroes, flushes and re-reads a SCHED_BINS histogram, so a block must own many more rows
+// than bins for that fixed cost to vanish (at 512 rows it was 8 bins per row)
+static constexpr int SCHED_CHUNK = 4096;
 __device__ __forceinline__ int tile_bin(int tm) {
     const int m = tm & 0x7ffffff;
     return m ? ((tm >> 27) & 15) * 28 + (27 - __popc(m)) : 511;
@@ -329,26 +453,29 @@ __global__ void __launch_bounds__(256) k_sched_scatter(const int32_t* __restrict
                                                        const uint16_t* __restrict__ keys, int* __restrict__ offs, int* __restrict__ tile_mask,
                                                        int* __restrict__ ticket, int32_t* __restrict__ order, int fb) {
     // block-aggregated counting-sort scatter: count this block's rows per digest in shared memory, reserve one global range
-    // per (block, digest) with a single atomic, then hand out positions from shared memory
+    // per (block, digest) with a single atomic, then hand out positions from shared memory.  The grid is sized by the
+    // capacity (no host read of the count); blocks past the count only take their ticket.
     __shared__ int s_cnt[SCHED_BINS];
     const int n = min(*d_n, cap);
     const int r0 = blockIdx.x * SCHED_CHUNK, r1 = min(n, r0 + SCHED_CHUNK);
-    for (int b = threadIdx.x; b < SCHED_BINS; b += blockDim.x) s_cnt[b] = 0;
-    __syncthreads();
-    for (int i = r0 + threadIdx.x; i < r1; i += blockDim.x) atomicAdd(s_cnt + keys[i], 1);
-    __syncthreads();
-    for (int b = threadIdx.x; b < SCHED_BINS; b += blockDim.x) {
-        const int c = s_cnt[b];
-        if (c) s_cnt[b] = atomicAdd(offs + b, c);
-    }
-    __syncthreads();
-    for (int i = r0 + threadIdx.x; i < r1; i += blockDim.x) {
-        const int pos = atomicAdd(s_cnt + keys[i], 1);
-        order[pos] = i;
-        int m = __ldg(masks + i);
-        int* tm = tile_mask + (pos >> 7);
-        if (fb && (pos & 127) == 0) m |= (int)(keys[i] >> (12 - fb)) << 27;      // the tile's frame group = its first row's (bits 27..30)
-        if ((__ldcg(tm) & m) != m) atomicOr(tm, m);              // plain read first: after a few rows the tile's mask is complete
+    if (r0 < r1) {
+        for (int b = threadIdx.x; b < SCHED_BINS; b += blockDim.x) s_cnt[b] = 0;
+        __syncthreads();
+        for (int i = r0 + threadIdx.x; i < r1; i += blockDim.x) atomicAdd(s_cnt + keys[i], 1);
+        __syncthreads();
+        for (int b = threadIdx.x; b < SCHED_BINS; b += blockDim.x) {
+            const int c = s_cnt[b];
+            if (c) s_cnt[b] = atomicAdd(offs + b, c);
+        }
+        __syncthreads();
+        for (int i = r0 + threadIdx.x; i < r1; i += blockDim.x) {
+            const int pos = atomicAdd(s_cnt + keys[i], 1);
+            order[pos] = i;
+            int m = __ldg(masks + i);
+            int* tm = tile_mask + (pos >> 7);
+            if (fb && (pos & 127) == 0) m |= (int)(keys[i] >> (12 - fb)) << 27;      // the tile's frame group = its first row's (bits 27..30)
+            if ((__ldcg(tm) & m) != m) atomicOr(tm, m);              // plain read first: after a few rows the tile's mask is complete
+        }
     }
     // ---- the last block orders the tiles by descending work (counting sort over popc(mask) = 0..27)
     // frame-major: bin = frame group * 28 + (27 - live offsets); empty capacity tiles (mask 0) go last (bin 511)
@@ -356,10 +483,11 @@ __global__ void __launch_bounds__(256) k_sched_scatter(const int32_t* __restrict
     __threadfence();
     __syncthreads();
     if (threadIdx.x == 0) s_last = (atomicAdd(ticket, 1) == (int)gridDim.x - 1);
-    for (int b = threadIdx.x; b < 512; b += blockDim.x) bins[b] = 0;
     __syncthreads();
     if (!s_last) return;
+    for (int b = threadIdx.x; b < 512; b += blockDim.x) bins[b] = 0;
     __threadfence();
+    __syncthreads();
     const int tiles = (cap + 127) >> 7;
     int32_t* tile_order = order + cap;
     // warp-aggregated (28 bins, thousands of tiles: per-tile shared-memory atomics on the same few counters serialise)
@@ -371,9 +499,12 @@ __global__ void __launch_bounds__(256) k_sched_scatter(const int32_t* __restrict
         if (t < tiles && lane == __ffs(peers) - 1) atomicAdd(bins + bin, __popc(peers));
     }
     __syncthreads();
-    if (threadIdx.x == 0) {
-        int run = 0;
-        for (int b = 0; b < 512; ++b) { int c = bins[b]; bins[b] = run; run += c; }
+    {                                                                      // exclusive scan of the 512 bins, 2 per thread
+        const int c0 = bins[2 * threadIdx.x], c1 = bins[2 * threadIdx.x + 1];
+        int total;
+        const int run = block_exclusive_scan(c0 + c1, &total);
+        bins[2 * threadIdx.x] = run;
+        bins[2 * threadIdx.x + 1] = run + c0;
     }
     __syncthreads();
     for (int t0 = threadIdx.x - lane; t0 < tiles; t0 += blockDim.x) {
@@ -413,6 +544,93 @@ __global__ void __launch_bounds__(256) k_sched_tiles(const int32_t* __restrict__
             if (k < K) dst[k * 128] = w[k];
         dst[K * 128] = i;
     }
+}
+
+// direct path's tile pass: the same tile-major table as k_sched_tiles, but the ranks are computed here from the grid index
+// (no row-major table exists).  One thread per tile position p: row i = order[p], its coordinates and mask; for each LIVE
+// kernel line one or two bitmap words + prefix words give every tap's rank = prefix + popc (grid_lookup's arithmetic),
+// then perm.  Plane k is written coalesced across the warp.
+__global__ void __launch_bounds__(256) k_tiles_direct(const int32_t* __restrict__ coords, int cap, const int* __restrict__ d_n, ConvGeom cg,
+                                                      GridIndex g, int centre, const int* __restrict__ masks, const int32_t* __restrict__ order,
+                                                      const int* __restrict__ tile_mask, int32_t* __restrict__ tab_tiles) {
+    const int n = min(*d_n, cap);
+    const int tiles_n = (n + 127) >> 7;
+    const int tiles = (cap + 127) >> 7;
+    const int K = cg.k[0] * cg.k[1] * cg.k[2];
+    int32_t* mask_out = const_cast<int32_t*>(order) + cap + tiles;                 // order[cap + tiles + j] = OR of tile j's row masks
+    for (int j = blockIdx.x * blockDim.x + threadIdx.x; j < tiles; j += gridDim.x * blockDim.x) mask_out[j] = __ldg(tile_mask + j) & 0x7ffffff;
+    for (int pos = blockIdx.x * blockDim.x + threadIdx.x; pos < tiles_n * 128; pos += gridDim.x * blockDim.x) {
+        const int i = pos < n ? __ldg(order + pos) : -1;
+        int4 c = make_int4(0, 0, 0, 0);
+        uint32_t m = 0;                                                            // no live tap beyond the count
+        if (i >= 0) { c = __ldg(reinterpret_cast<const int4*>(coords) + i); m = (uint32_t)__ldg(masks + i); }
+        const int z0 = c.y * cg.s[0] - cg.p[0], y0 = c.z * cg.s[1] - cg.p[1], x0 = c.w * cg.s[2] - cg.p[2];
+        int32_t* dst = tab_tiles + (size_t)(pos >> 7) * (K + 1) * 128 + (pos & 127);
+#pragma unroll
+        for (int kz = 0; kz < 3; ++kz)
+#pragma unroll
+            for (int ky = 0; ky < 3; ++ky) {
+                if (kz >= cg.k[0] || ky >= cg.k[1]) continue;
+                const int line = kz * cg.k[1] + ky;
+                const uint32_t lm = (m >> (line * cg.k[2])) & ((1u << cg.k[2]) - 1u);
+                LineWords l{0, 0, 0, 0, 0};
+                uint32_t p_lo = 0, p_hi = 0;
+                if (lm) {                                                          // live line: its words and prefixes
+                    l = line_words(g, c.x, z0 + kz, y0 + ky, x0, cg.k[2]);
+                    const size_t wi = (size_t)(l.c_lo >> 5);
+                    p_lo = __ldg(g.prefix + wi);
+                    p_hi = (l.c_lo & 31) + l.n > 32 ? __ldg(g.prefix + wi + 1) : p_lo;      // the line spans two words
+                }
+#pragma unroll
+                for (int kx = 0; kx < 3; ++kx) {
+                    if (kx >= cg.k[2]) continue;
+                    const int k = line * cg.k[2] + kx;
+                    int v = -1;
+                    if ((lm >> kx) & 1u) {
+                        if (k == centre) {
+                            v = i;                                                 // the site itself
+                        } else {
+                            const int bit = (int)(l.c_lo & 31) + (kx - l.x_lo);    // live => inside the clipped range
+                            const uint32_t word = bit < 32 ? l.w_lo : l.w_hi;
+                            const int rank = (int)((bit < 32 ? p_lo : p_hi) + __popc(word & ((1u << (bit & 31)) - 1u)));
+                            v = g.perm ? __ldg(g.perm + rank) : rank;
+                        }
+                    }
+                    dst[k * 128] = v;
+                }
+            }
+        dst[K * 128] = i;
+    }
+}
+
+extern "C" int dz_rulebook_schedule_direct(const int32_t* coords, int cap, const int* d_n, int B, const int* in_dhw, const int* ks,
+                                           const int* st_, const int* pd, int subm, const uint32_t* in_bitmap, const uint32_t* in_prefix,
+                                           const int32_t* in_perm, int32_t* order, void* sched_ws, size_t ws_bytes, int sched_frame_major,
+                                           int32_t* tab_tiles, dz_stream_t stream) {
+    DZ_CHECK_ARG(coords && d_n && in_bitmap && in_prefix && order && sched_ws && tab_tiles && cap >= 1 && B >= 1);
+    if (ws_bytes < dz_rulebook_schedule_ws_bytes(cap)) { dz_set_error("dz_rulebook_schedule_direct: workspace too small"); return DZ_ERR_WORKSPACE; }
+    ConvGeom cg;
+    if (subm) {
+        DZ_CHECK_ARG(ks[0] % 2 == 1 && ks[1] % 2 == 1 && ks[2] % 2 == 1 && ks[0] <= 3 && ks[1] <= 3 && ks[2] <= 3);
+        cg = subm_geom(in_dhw[0], in_dhw[1], in_dhw[2], ks);
+    } else {
+        for (int d = 0; d < 3; ++d) {
+            DZ_CHECK_ARG(ks[d] >= 1 && ks[d] <= 3 && st_[d] >= 1 && pd[d] >= 0);
+            cg.k[d] = ks[d]; cg.s[d] = st_[d]; cg.p[d] = pd[d]; cg.in_dhw[d] = in_dhw[d];
+            cg.out_dhw[d] = (in_dhw[d] + 2 * pd[d] - (ks[d] - 1) - 1) / st_[d] + 1;
+        }
+    }
+    const int K = cg.k[0] * cg.k[1] * cg.k[2];
+    cudaStream_t st = (cudaStream_t)stream;
+    TableOut to = table_out(nullptr, nullptr, sched_ws, cap);
+    k_sched_scatter<<<dz_cdiv(cap, SCHED_CHUNK), 256, 0, st>>>(to.masks, cap, d_n, to.keys, to.hist, to.hist + SCHED_BINS, to.ticket + 1, order,
+                                                                sched_frame_bits(B, sched_frame_major));
+    DZ_LAUNCH_CHECK();
+    GridIndex g{in_bitmap, in_prefix, in_perm, B, in_dhw[0], in_dhw[1], in_dhw[2], dz_cells_pad(in_dhw[0], in_dhw[1], in_dhw[2])};
+    const int blocks = max(1, min(dz_cdiv(cap, 256), DZ_NUM_SMS * 8));
+    k_tiles_direct<<<blocks, 256, 0, st>>>(coords, cap, d_n, cg, g, subm ? (K - 1) / 2 : -1, to.masks, order, to.hist + SCHED_BINS, tab_tiles);
+    DZ_LAUNCH_CHECK();
+    return DZ_OK;
 }
 
 extern "C" int dz_rulebook_schedule(const int32_t* tab, int cap, const int* d_n, int32_t* order, void* sched_ws, size_t ws_bytes,

@@ -560,7 +560,10 @@ extern "C" int dz_spconv_fwd_planes(const void* in, int cin, int in_rows, const 
                                     const int* d_n_out, int out_cap, const void* weight, const float* scale, const float* shift,
                                     const void* residual, int relu, void* out, int cout, int planes, const int32_t* tab_tiles,
                                     dz_stream_t stream) {
-    DZ_CHECK_ARG(in && tab && d_n_out && weight && out && cin >= 1 && K >= 1 && K <= SB_KMAX && out_cap >= 1 && tab_rows >= out_cap);
+    // tab may be NULL when the tile-major table and its schedule are given (the direct rulebook path builds no row-major table);
+    // tab_rows is then the rulebook's capacity, which sizes `row_order`
+    DZ_CHECK_ARG(in && (tab || (tab_tiles && row_order)) && d_n_out && weight && out && cin >= 1 && K >= 1 && K <= SB_KMAX && out_cap >= 1 &&
+                 tab_rows >= out_cap);
     DZ_CHECK_ARG(planes == 1 || planes == 2);
     (void)in_rows;
     cudaStream_t st = (cudaStream_t)stream;

@@ -199,6 +199,69 @@ def rulebook_schedule(tab, d_n, sched_ws, B=1, frame_major=False, K=None):
     return order, tab_tiles
 
 
+def rulebook_subm_masks(coords, d_n, cap, index, ksize, sched_ws, frame_major=False, perm_walk=True):
+    """direct path (bf16-plane layers with a schedule), mask pass of a submanifold rulebook: fills sched_ws as rulebook_subm
+    does and writes no table; rulebook_schedule_direct then builds the tile-major table.  perm_walk: visit the rows in lattice
+    order through the index's perm (ignored without one)"""
+    _need_cuda(coords)
+    walk = bool(perm_walk) and index.perm is not None
+    check(lib().dz_rulebook_subm_masks(_p(coords), _p(d_n), cap, index.B, *index.dhw, iarr(ksize), _p(index.bitmap), _p(index.prefix),
+                                       _p(index.perm), _p(sched_ws), int(bool(frame_major)), int(walk), _stream()), 'rulebook_subm_masks')
+    _count(2)
+
+
+def rulebook_conv_masks(coords, d_n, in_cap, in_index, ksize, stride, pad, out_cap, sched_ws, frame_major=False):
+    """direct path, mask pass of a strided-conv rulebook: the output sites, their count and grid index as rulebook_conv, and
+    sched_ws filled as rulebook_conv fills it; no table.  Returns (out_coords, d_n_out, out_index, out_dhw)"""
+    _need_cuda(coords)
+    dev = coords.device
+    out_dhw = conv_out_dhw(in_index.dhw, ksize, stride, pad)
+    out_index = GridIndex(in_index.B, out_dhw, dev)
+    out_coords = torch.empty((out_cap, 4), dtype=torch.int32, device=dev)
+    d_n_out = torch.empty(1, dtype=torch.int32, device=dev)
+    ws = workspace(scan_ws_bytes(out_index.words), dev, 'rulebook')
+    check(lib().dz_rulebook_conv_masks(_p(coords), _p(d_n), in_cap, in_index.B, iarr(in_index.dhw), iarr(ksize), iarr(stride), iarr(pad),
+                                       _p(in_index.bitmap), _p(in_index.prefix), _p(in_index.perm), _p(out_coords), _p(d_n_out), out_cap,
+                                       _p(out_index.bitmap), _p(out_index.prefix), _p(ws), ws.numel(), _p(sched_ws), int(bool(frame_major)),
+                                       _stream()), 'rulebook_conv_masks')
+    _count(7)
+    return out_coords, d_n_out, out_index, out_dhw
+
+
+def rulebook_schedule_direct(coords, d_n, cap, in_index, ksize, stride, pad, subm, sched_ws, B=1, frame_major=False):
+    """direct path: schedule + tile-major table of a rulebook whose mask pass filled sched_ws.  coords / d_n / cap: the rulebook's
+    rows (output sites); in_index: the grid index of the conv's input.  Returns (order, tab_tiles) as rulebook_schedule(K=...)"""
+    _need_cuda(coords)
+    K = ksize[0] * ksize[1] * ksize[2]
+    tiles = (cap + 127) // 128
+    order = torch.empty(cap + 2 * tiles, dtype=torch.int32, device=coords.device)
+    tab_tiles = torch.empty((tiles, K + 1, 128), dtype=torch.int32, device=coords.device)
+    check(lib().dz_rulebook_schedule_direct(_p(coords), cap, _p(d_n), int(B), iarr(in_index.dhw), iarr(ksize), iarr(stride), iarr(pad),
+                                            int(bool(subm)), _p(in_index.bitmap), _p(in_index.prefix), _p(in_index.perm), _p(order),
+                                            _p(sched_ws), sched_ws.numel(), int(bool(frame_major)), _p(tab_tiles), _stream()),
+          'rulebook_schedule_direct')
+    _count(2)
+    return order, tab_tiles
+
+
+def tiles_to_rows(tab_tiles, order, d_n, cap):
+    """tile-major table + its schedule -> the row-major (cap, 32) table in canonical row order (rows beyond the count: -1,
+    mask 0).  For callers that need the row form of a direct-path rulebook; no host read of the count"""
+    tiles, K1, _ = tab_tiles.shape
+    K = K1 - 1
+    dev = tab_tiles.device
+    flat = tab_tiles.permute(0, 2, 1).reshape(tiles * 128, K1)
+    pos = torch.arange(tiles * 128, device=dev)
+    live = (pos < d_n.long()) & (pos < cap)
+    dst = torch.where(live, flat[:, K].long(), torch.full_like(pos, cap))       # positions beyond the count go to a spare row
+    tab = torch.full((cap + 1, 32), -1, dtype=torch.int32, device=dev)
+    tab[dst, :K] = flat[:, :K]
+    tab = tab[:cap]
+    tab[:, 27] = ((tab[:, :K] >= 0).to(torch.int64) << torch.arange(K, device=dev)[None, :]).sum(1).to(torch.int32)
+    tab[:, 28:] = 0
+    return tab
+
+
 def table_to_rows(nbr):
     """k-major (K, cap) table -> the row-major (cap, 32) layout of the tensor-core kernels (host-side helper for callers that
     only hold the k-major form; the rulebook kernels write either layout directly)"""
@@ -267,17 +330,23 @@ def spconv_fwd(feats, nbr, d_n_out, out_cap, weight_packed, scale, shift, residu
     """feats (in_cap, cin); weight_packed per pack_spconv_weight; kshape = (K, cin, cout).
     nbr: k-major (K, cap) table for DZ_F32; row-major (cap, 32) table for the tensor-core modes (a k-major table is
     converted on the fly); layout: 'k' | 'row' says which one `nbr` is (None: inferred from the shape, ambiguous only for
-    cap == K or cap == 32 -- callers that know pass it); row_order: tile schedule from rulebook_schedule (tensor-core modes)"""
+    cap == K or cap == 32 -- callers that know pass it); row_order: tile schedule from rulebook_schedule (tensor-core modes).
+    nbr may be None for the bf16-plane modes when tab_tiles and row_order are given (direct-path rulebook: no row-major table)"""
     _need_cuda(feats, nbr, weight_packed)
     K, cin, cout = kshape if kshape is not None else weight_packed.shape
-    if layout is None:
+    if nbr is None:
+        if not (_lib.PLANES.get(mode) and tab_tiles is not None and row_order is not None):
+            raise RuntimeError('spconv_fwd without a row-major table needs a bf16-plane mode, tab_tiles and row_order')
+        assert row_order.numel() == out_cap + 2 * tab_tiles.shape[0] and tab_tiles.shape[1] == K + 1
+    elif layout is None:
         layout = 'row' if (nbr.shape[1] == 32 and nbr.shape[0] != K) else 'k'
-    assert layout in ('k', 'row')
-    if mode != _lib.DZ_F32 and layout == 'k':
-        nbr = table_to_rows(nbr)
-    elif mode == _lib.DZ_F32 and layout == 'row':
-        raise RuntimeError('the exact-fp32 kernel needs the k-major (K, cap) table')
-    assert nbr.shape[0] == K if mode == _lib.DZ_F32 else nbr.shape[1] == 32
+    if nbr is not None:
+        assert layout in ('k', 'row')
+        if mode != _lib.DZ_F32 and layout == 'k':
+            nbr = table_to_rows(nbr)
+        elif mode == _lib.DZ_F32 and layout == 'row':
+            raise RuntimeError('the exact-fp32 kernel needs the k-major (K, cap) table')
+        assert nbr.shape[0] == K if mode == _lib.DZ_F32 else nbr.shape[1] == 32
     planes = _lib.PLANES.get(mode, 0)
     if planes:
         cin_pad = 8 if cin <= 8 else cin
@@ -294,7 +363,8 @@ def spconv_fwd(feats, nbr, d_n_out, out_cap, weight_packed, scale, shift, residu
         ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         ev0.record()
     if planes:
-        check(lib().dz_spconv_fwd_planes(_p(feats), cin, feats.shape[0], _p(nbr), K, nbr.shape[0], _p(row_order), _p(d_n_out), out_cap,
+        check(lib().dz_spconv_fwd_planes(_p(feats), cin, feats.shape[0], _p(nbr), K, out_cap if nbr is None else nbr.shape[0], _p(row_order),
+                                         _p(d_n_out), out_cap,
                                          _p(weight_packed), _p(scale), _p(shift), _p(residual), int(relu), _p(out), cout, planes,
                                          _p(tab_tiles if row_order is not None else None), _stream()), 'spconv_fwd_planes')
     else:
@@ -308,6 +378,8 @@ def spconv_fwd(feats, nbr, d_n_out, out_cap, weight_packed, scale, shift, residu
         torch.cuda.synchronize()
         n_out = min(int(d_n_out.item()), out_cap)
         n_in = min(int(d_n_in.item()), feats.shape[0]) if d_n_in is not None else n_out
+        if nbr is None:                                 # direct-path rulebook: the trace records the row-major form (outside the events)
+            nbr = tiles_to_rows(tab_tiles, row_order, d_n_out, out_cap)
         _trace.append(dict(start=ev0, end=ev1, K=K, cin=cin, cout=cout, n_in=n_in, n_out=n_out, nbr=nbr, row_order=row_order,
                            residual=residual is not None))
     return out

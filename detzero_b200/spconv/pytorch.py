@@ -219,7 +219,12 @@ class _SparseConv(SparseModule):
     #: build a tile schedule (rows grouped by neighbour mask) with every rulebook used by a tensor-core layer
     SCHEDULE_TILES = True
     #: batches: sort the schedule by (frame, mask) so that the tiles in flight gather from ONE frame's (L2-resident) feature map
-    FRAME_MAJOR = bool(os.environ.get('DZ_FRAME_MAJOR'))      # measured (profiles/r02_spconv_notes.md): the 3 digest bits it costs outweigh the L2 gain
+    FRAME_MAJOR = bool(int(os.environ.get('DZ_FRAME_MAJOR', '0')))      # measured (profiles/r02_spconv_notes.md): the 3 digest bits it costs outweigh the L2 gain
+    #: bf16-plane layers with a schedule: build the tile-major table directly from the grid index (mask pass -> scatter -> tile
+    #: pass) instead of writing a row-major table and transposing it; the tables are identical row for row
+    DIRECT_TILES = True
+    #: direct path, submanifold mask pass: visit rows in lattice order (neighbouring lanes share bitmap lines)
+    MASK_PERM_WALK = True
 
     def __init__(self, in_channels, out_channels, kernel_size, stride=1, padding=0, dilation=1, groups=1, bias=True,
                  indice_key=None, subm=False, algo=None, mode='fp32'):
@@ -255,12 +260,19 @@ class _SparseConv(SparseModule):
             tc = _lib.MODES[self.mode] != _lib.DZ_F32
             layout = 'row' if tc else 'k'
             want = self._wants_schedule()
+            direct = want and self.DIRECT_TILES and _lib.MODES[self.mode] in _lib.PLANES
             fm = self.FRAME_MAJOR and x.batch_size > 1
             if self.subm:
                 sws = ops.new_sched_ws(x._cap, x._idx.device) if want else None
-                t = ops.rulebook_subm(x._idx, x._count, x._cap, x.grid_index(), self.kernel_size, layout=layout, sched_ws=sws,
-                                      frame_major=fm)
-                rule = _RuleSubm(None if tc else t, t if tc else None)
+                if direct:
+                    ops.rulebook_subm_masks(x._idx, x._count, x._cap, x.grid_index(), self.kernel_size, sws, frame_major=fm,
+                                            perm_walk=self.MASK_PERM_WALK)
+                    rule = _RuleSubm(None, None)
+                else:
+                    t = ops.rulebook_subm(x._idx, x._count, x._cap, x.grid_index(), self.kernel_size, layout=layout, sched_ws=sws,
+                                          frame_major=fm)
+                    rule = _RuleSubm(None if tc else t, t if tc else None)
+                rule.rows = (x._idx, x._count, x._cap)
             else:
                 in_index = x.grid_index()
                 out_dhw = ops.conv_out_dhw(x.spatial_shape, self.kernel_size, self.stride, self.padding)
@@ -276,11 +288,18 @@ class _SparseConv(SparseModule):
                 if hint is not None:
                     out_cap = int(min(cells, max(128, (int(hint * self.CAP_HEADROOM) + 127) // 128 * 128)))
                 sws = ops.new_sched_ws(out_cap, x._idx.device) if want else None
-                oc, d_n_out, out_index, t, odhw = ops.rulebook_conv(x._idx, x._count, x._cap, in_index, self.kernel_size, self.stride,
-                                                                    self.padding, out_cap, layout=layout, sched_ws=sws, frame_major=fm)
-                rule = _RuleConv(oc, d_n_out, out_index, (None, t) if tc else (t, None), odhw, out_cap)
+                if direct:
+                    oc, d_n_out, out_index, odhw = ops.rulebook_conv_masks(x._idx, x._count, x._cap, in_index, self.kernel_size, self.stride,
+                                                                           self.padding, out_cap, sws, frame_major=fm)
+                    rule = _RuleConv(oc, d_n_out, out_index, (None, None), odhw, out_cap)
+                else:
+                    oc, d_n_out, out_index, t, odhw = ops.rulebook_conv(x._idx, x._count, x._cap, in_index, self.kernel_size, self.stride,
+                                                                        self.padding, out_cap, layout=layout, sched_ws=sws, frame_major=fm)
+                    rule = _RuleConv(oc, d_n_out, out_index, (None, t) if tc else (t, None), odhw, out_cap)
+                rule.rows = (oc, d_n_out, out_cap)
             rule.sched_ws = sws
             rule.frame_major = fm
+            rule.direct = direct
             rule.in_idx, rule.in_count, rule.in_cap, rule.in_dhw, rule.in_index = x._idx, x._count, x._cap, x.spatial_shape, x._index
             if key is not None:
                 x.indice_dict[key] = rule
@@ -297,14 +316,24 @@ class _SparseConv(SparseModule):
         if rule.order is None and rule.sched_ws is not None:
             d_n = x._count if self.subm else rule.d_n_out
             fm = getattr(rule, 'frame_major', False)
-            if _lib.MODES[self.mode] in _lib.PLANES:        # persistent kernel: also the tile-major table (one bulk copy per tile)
+            if getattr(rule, 'direct', False):             # tile-major table straight from the masks and the input grid index
+                rows, d_n, cap = rule.rows
+                stride, pad = ([1, 1, 1], [0, 0, 0]) if self.subm else (self.stride, self.padding)
+                rule.order, rule.tab_tiles = ops.rulebook_schedule_direct(rows, d_n, cap, rule.in_index, self.kernel_size, stride, pad,
+                                                                          self.subm, rule.sched_ws, x.batch_size, fm)
+            elif _lib.MODES[self.mode] in _lib.PLANES:        # persistent kernel: also the tile-major table (one bulk copy per tile)
                 rule.order, rule.tab_tiles = ops.rulebook_schedule(rule.tab, d_n, rule.sched_ws, x.batch_size, fm, K=self.kshape[0])
             else:
                 rule.order = ops.rulebook_schedule(rule.tab, d_n, rule.sched_ws, x.batch_size, fm)
 
     def _table(self, rule):
-        """(table, row_order) for this layer's kernel"""
+        """(table, row_order) for this layer's kernel; the table is None for a direct-path rulebook on a bf16-plane layer"""
         if _lib.MODES[self.mode] != _lib.DZ_F32:
+            if rule.tab is None and rule.nbr is None:     # direct path: only the tile-major table exists
+                if _lib.MODES[self.mode] in _lib.PLANES:
+                    return None, rule.order
+                _, d_n, cap = rule.rows
+                rule.tab = ops.tiles_to_rows(rule.tab_tiles, rule.order, d_n, cap)
             if rule.tab is None:                      # rulebook shared with an exact-fp32 layer: convert once
                 rule.tab = ops.table_to_rows(rule.nbr)
             return rule.tab, rule.order
@@ -448,6 +477,8 @@ class SparseInverseConv3d(SparseModule):
             raise RuntimeError('SparseInverseConv3d(%r): no SparseConv3d with this indice_key has run on this tensor' % self.indice_key)
         K = self.kernel_size[0] * self.kernel_size[1] * self.kernel_size[2]
         if rule.nbr is None:                                    # rulebook built for a tensor-core layer: k-major copy of the row-major table
+            if rule.tab is None:                                # direct path: row-major form of the tile-major table first
+                rule.tab = ops.tiles_to_rows(rule.tab_tiles, rule.order, rule.d_n_out, rule.out_cap)
             rule.nbr = rule.tab[:, :K].t().contiguous()
         if not hasattr(rule, 'in_idx'):
             raise RuntimeError('rulebook %r does not remember its input sites' % self.indice_key)

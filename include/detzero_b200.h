@@ -133,6 +133,32 @@ int dz_rulebook_schedule(const int32_t* tab, int cap, const int* d_n, int32_t* o
  * count).  With it `order` must have cap + 2*ceil(cap/128) ints: order[cap + tiles + j] = OR of tile j's row masks.  The
  * persistent bf16-plane conv (dz_spconv_fwd_planes) fetches a tile's block with ONE bulk copy. */
 
+/* Direct path to tab_tiles without a row-major table (the schedule + tile-major table of the bf16-plane conv; same pair set as
+ * spconv's generate_subm_conv_inds / generate_conv_inds_stage{1,2}).  Two calls per rulebook:
+ *   1. dz_rulebook_subm_masks / dz_rulebook_conv_masks: the mask pass.  Leaves in sched_ws exactly what dz_rulebook_subm /
+ *      dz_rulebook_conv leave there (neighbour masks, digests, scanned histogram) and writes no table.  The strided variant
+ *      also produces the output sites, their count and their grid index, as dz_rulebook_conv does.  perm_walk (needs perm):
+ *      visit the rows in lattice (rank) order.
+ *   2. dz_rulebook_schedule_direct: the schedule and the tile-major table from the masks and the INPUT grid index.  coords,
+ *      cap, d_n are the OUTPUT sites (the rulebook's rows); in_dhw3 / ksize3 / stride3 / pad3 the conv geometry; subm = 1 for a
+ *      submanifold conv (stride and pad are then ignored: 1 and (k-1)/2).  order: cap + 2*ceil(cap/128) ints and tab_tiles:
+ *      ceil(cap/128) * (K+1) * 128 ints, both as dz_rulebook_schedule with K given.  Plane k of every row equals the entry
+ *      the row-major table would hold. */
+int dz_rulebook_subm_masks(const int32_t* coords, const int* d_n, int cap, int B, int D, int H, int W,
+                           const int* ksize3_host, const uint32_t* bitmap, const uint32_t* prefix, const int32_t* perm,
+                           void* sched_ws, int sched_frame_major, int perm_walk, dz_stream_t stream);
+int dz_rulebook_conv_masks(const int32_t* in_coords, const int* d_n_in, int in_cap, int B,
+                           const int* in_dhw3_host, const int* ksize3_host, const int* stride3_host,
+                           const int* pad3_host, const uint32_t* in_bitmap, const uint32_t* in_prefix,
+                           const int32_t* in_perm, int32_t* out_coords, int* d_n_out, int out_cap,
+                           uint32_t* out_bitmap, uint32_t* out_prefix, void* ws, size_t ws_bytes,
+                           void* sched_ws, int sched_frame_major, dz_stream_t stream);
+int dz_rulebook_schedule_direct(const int32_t* coords, int cap, const int* d_n, int B, const int* in_dhw3_host,
+                                const int* ksize3_host, const int* stride3_host, const int* pad3_host, int subm,
+                                const uint32_t* in_bitmap, const uint32_t* in_prefix, const int32_t* in_perm,
+                                int32_t* order, void* sched_ws, size_t ws_bytes, int sched_frame_major,
+                                int32_t* tab_tiles, dz_stream_t stream);
+
 /* ---- sparse convolution -------------------------------------------------------------------------------- */
 /* out[o,:] = act( (sum_k in[nbr[k][o],:] @ W[k]) * scale + shift (+ residual[o,:]) )
  * Replaces SubMConv3d/SparseConv3d forward + BatchNorm1d(eval) + bias + residual add + ReLU
@@ -159,7 +185,8 @@ int dz_spconv_wgrad(const float* in, int cin, const int32_t* nbr, int K, int nbr
  * warp-specialised tcgen05 kernel.  Feature tensors `in`, `residual`, `out` are (rows, planes * C) bf16, a row = [p0 | p1] with
  * x ~ p0 (+ p1), p0 = RN_bf16(x), p1 = RN_bf16(x - p0); cin <= 8 is stored padded to 8 channels per plane.  weight: (planes * cout,
  * K * cin_pad) bf16, rows [w0 ; w1] split the same way.  tab = ROW-major table, row_order = NULL or the tile schedule,
- * tab_tiles = NULL or the tile-major table dz_rulebook_schedule wrote next to row_order (fast path).
+ * tab_tiles = NULL or the tile-major table dz_rulebook_schedule wrote next to row_order (fast path).  With tab_tiles and
+ * row_order, tab may be NULL (direct rulebook path); tab_rows is then the rulebook's capacity.
  * No reference counterpart for the storage format (spconv keeps fp32 rows); dz_to_planes / dz_from_planes convert at the
  * boundary: out[r, p, 0..c_pad) <- x[r, 0..c) (zero padded), x[r, c] <- p0 + p1. */
 int dz_spconv_fwd_planes(const void* in, int cin, int in_rows, const int32_t* tab, int K, int tab_rows,
